@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py — the discovery-scan benchmark (contract: see the task statement / DESIGN.md §Measurement).
 
-  python bench.py [--gpus N --steps K --warmup W] [--impl reference] [--records R]
+  python bench.py [--gpus N --steps K --warmup W] [--impl reference] [--records R] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch of synthetic input:
   parse the full utils/pci.ids image (1,536,458 B) into the name table  +  classify / compact /
@@ -16,6 +16,10 @@ value   records/s with inputs resident in HBM (CUDA events on the launching stre
         between steps, max over ranks)
 e2e     the same metric through the reference-facing C-ABI calls (kvg_pciids_load + kvg_scan_pci)
         with PINNED HOST buffers in and host results out, copies inside the timed region
+
+--dump-outputs DIR writes the result of the last timed step, as a caller of the scan receives it, to
+DIR/<name>.npy (float64, one file per array; N > 1: every rank its own part, prefixed rank<r>_).  The
+inputs depend on the arguments only, so two builds can be compared array for array.
 """
 import argparse
 import gzip
@@ -180,6 +184,47 @@ def check_parity(ctx, sharded, rank, world, n, ids, gbits, text, O):
             "survivors_global": int(len(addr))}
 
 
+DUMP_BYTES = 60_000_000   # array data of one --dump-outputs run: under 64 MB with the .npy headers
+
+
+def result_arrays(res, prefix="", maps=("dev", "grp")):
+    """The arrays of a PciResult: one per survivor field, the orderings of `maps`, and with the device-id
+    ordering the name slots and the name pool they point into."""
+    out = {prefix + "survivors_" + f: res.survivors[f] for f in res.survivors.dtype.names}
+    for m in maps:
+        for f in ("keys", "off", "perm") + (("name_slot",) if m == "dev" else ()):
+            out["%s%s_%s" % (prefix, m, f)] = getattr(res, "%s_%s" % (m, f))
+    if "dev" in maps:
+        out[prefix + "name_pool"] = np.frombuffer(res.name_pool, dtype=np.uint8)
+    return out
+
+
+def last_step_arrays(ctx, sharded, rank):
+    """What the last scan handed its caller: the fetched result (N = 1), or this rank's part of the sharded
+    result (its shard's survivors and the members and orderings of the keys it owns)."""
+    if sharded is None:
+        return result_arrays(ctx.dev_scan_pci_fetch())
+    res = sharded.fetch()
+    out = {"local_" + f: res.local[f] for f in res.local.dtype.names}
+    out.update(result_arrays(res.dev, "devmap_", ("dev",)))
+    out.update(result_arrays(res.grp, "grpmap_", ("grp",)))
+    return {"rank%d_%s" % (rank, k): v for k, v in out.items()}
+
+
+def dump_outputs(out_dir, arrays, budget):
+    """One float64 .npy per array (exact for every integer the scan returns).  Past `budget` bytes in all,
+    every array keeps the same fraction of its elements, at indices drawn from a fixed seed, so two builds
+    that compute the same result write the same files."""
+    os.makedirs(out_dir, exist_ok=True)
+    total = 8 * sum(a.size for a in arrays.values())
+    keep = budget / total if total > budget else 1.0
+    for name, a in arrays.items():
+        a = np.ascontiguousarray(a, dtype=np.float64)
+        if keep < 1.0:
+            a = a[np.sort(np.random.default_rng(0).choice(a.size, int(a.size * keep), replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_reference(args, rank, world):
     """--impl reference: the reference's own CPU algorithm (oracle port; the Go binary cannot be
     built in this image) on the host cores, bounded sample per step."""
@@ -242,7 +287,13 @@ def main():
                     help="records for the HBM-bound roofline leg (N=1 only; 0 disables)")
     ap.add_argument("--big-files", type=int, default=256,
                     help="pci.ids images for the HBM-bound parse roofline leg (0 disables)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the result of the last timed step to DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the GPU scan's result; the reference arm has none")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -344,6 +395,8 @@ def main():
     launches = ctx.launch_count - launches0 - args.steps  # minus the flush fills
     dev_ms = sum(a.elapsed_time(b) for a, b in evs)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last_step_arrays(ctx, sharded, rank), DUMP_BYTES // world)
     if world > 1:
         t = torch.tensor([dev_ms], dtype=torch.float64, device="cuda")
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
