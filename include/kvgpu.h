@@ -14,6 +14,8 @@
  *                                            (+ readVgpuIDFromFileFunc label rule :334-344, join :152-155)
  *   kvg_health_rescan                     <- health flips fed to ListAndWatch
  *                                            generic_device_plugin.go:325-342, :611-690
+ *   kvg_rescan_pci, kvg_rescan_mdev       <- (no reference equivalent: the reference scans once at start-up,
+ *                                            device_plugin.go:89-96)
  *   kvg_comm_*, kvg_scan_pci_sharded      <- (no reference equivalent; BASELINE.json config 4)
  *
  * Plain C: pointers + sizes only, no C++ types, no exceptions cross this boundary.
@@ -238,6 +240,54 @@ typedef struct kvg_health_delta {
   const uint32_t *changed; /* [n_changed] (record index << 1) | now_alive, ascending index */
 } kvg_health_delta;
 
+/* ---- rescans (runtime rediscovery) -----------------------------------------------------------
+ * A rescan is a full scan of a fresh snapshot, diffed ON THE DEVICE against the previous successful rescan of
+ * the same kind on the same context (its baseline).
+ *
+ * Identity: a survivor is identified by `addr` (PCI) or by its 16 uuid bytes compared as a big-endian string
+ * (mdev).  The survivors of a snapshot must be strictly ascending in that identity, which is Walk order in
+ * numeric mode; the device checks it, and a violation returns KVG_EINVAL and keeps the baseline.  Snapshots in
+ * index mode (addresses / uuids that are Walk indices, interned groups, devices or parents) have no stable
+ * identity; the library cannot detect them and they must not be passed here.
+ *
+ * moved: identity in both lists, a map-relevant field differs (PCI: iommu_group, device, numa; mdev: type_key,
+ * parent, numa; name_slot and src never count).
+ * changed key: present before and after, and its member list AS THAT MAP STORES IT differs.  deviceMap,
+ * iommuMap and vGpuMap store (addr|uuid, numa) in Walk order; gpuVgpuMap stores uuids only.  So a group-only
+ * move changes two iommuMap keys and no deviceMap key; a numa-only mdev move changes its vGpuMap key and no
+ * gpuVgpuMap key.
+ * Type ids: the `types` of kvg_rescan_mdev must start with the previous rescan's dictionary byte for byte (new
+ * raw names may only be appended), else KVG_EINVAL: canonical type ids are only stable under that rule.
+ * Resets: kvg_pciids_load and kvg_rescan_reset drop both baselines; the next rescan then reports every
+ * survivor and key as added.  Baselines are independent of kvg_scan_*, kvg_dev_* and the health state.
+ * The result is one library-owned block, freed with kvg_result_free. */
+typedef struct kvg_key_delta { /* one group-by map; every list ascending */
+  uint32_t n_added;   const uint32_t *added;   /* keys absent before, present now             */
+  uint32_t n_removed; const uint32_t *removed; /* keys present before, absent now             */
+  uint32_t n_changed; const uint32_t *changed; /* present before and now, member list differs */
+} kvg_key_delta;
+
+typedef struct kvg_pci_rescan {
+  kvg_pci_result scan;             /* identical to kvg_scan_pci on the same records */
+  uint32_t had_baseline;           /* 0: first rescan since a reset -> everything is "added" */
+  uint64_t n_added;   const uint32_t *added;       /* indices into scan.survivors, ascending */
+  uint64_t n_removed; const kvg_pci_surv *removed; /* previous survivors, ascending addr      */
+  uint64_t n_moved;   const uint32_t *moved;       /* indices into scan.survivors: same addr,
+                                                      iommu_group / device / numa changed    */
+  kvg_key_delta dev;               /* deviceMap, keys = device ids */
+  kvg_key_delta grp;               /* iommuMap,  keys = group ids  */
+} kvg_pci_rescan;
+
+typedef struct kvg_mdev_rescan {
+  kvg_mdev_result scan;            /* identical to kvg_scan_mdev */
+  uint32_t had_baseline;
+  uint64_t n_added;   const uint32_t *added;
+  uint64_t n_removed; const kvg_mdev_surv *removed;
+  uint64_t n_moved;   const uint32_t *moved;       /* same uuid, type_key / parent / numa changed */
+  kvg_key_delta type;              /* vGpuMap,    keys = canonical type ids */
+  kvg_key_delta parent;            /* gpuVgpuMap, keys = parent handles     */
+} kvg_mdev_rescan;
+
 /* ---- context -------------------------------------------------------------------------------- */
 typedef struct kvg_ctx kvg_ctx;
 
@@ -287,6 +337,12 @@ int kvg_scan_mdev(kvg_ctx *ctx, const kvg_mdev_rec *recs, size_t n, const kvg_ty
  * against "nothing alive").  n must stay constant between calls; kvg_health_reset() re-arms. */
 int kvg_health_rescan(kvg_ctx *ctx, const kvg_pci_rec *recs, size_t n, kvg_health_delta **delta);
 int kvg_health_reset(kvg_ctx *ctx);
+/* Scan `recs` exactly as kvg_scan_pci / kvg_scan_mdev do and diff the result against the baseline (see
+ * "rescans" above); on success the new scan becomes the baseline. */
+int kvg_rescan_pci(kvg_ctx *ctx, const kvg_pci_rec *recs, size_t n, kvg_pci_rescan **res);
+int kvg_rescan_mdev(kvg_ctx *ctx, const kvg_mdev_rec *recs, size_t n, const kvg_type_dict *types,
+                    kvg_mdev_rescan **res);
+int kvg_rescan_reset(kvg_ctx *ctx); /* drops both baselines */
 
 /* ---- device-resident entry points (inputs already in HBM; used by bench.py "value") -------- */
 

@@ -31,6 +31,7 @@
 #include "kvg_scan.cuh"
 #include "kvg_order.cuh"
 #include "kvg_shard.cuh"
+#include "kvg_rescan.cuh"
 
 using namespace kvg;
 
@@ -42,3 +43,4 @@ using namespace kvg;
 #include "api/kvg_api_mdev.inc"
 #include "api/kvg_api_util.inc"
 #include "api/kvg_api_shard.inc"
+#include "api/kvg_api_rescan.inc"

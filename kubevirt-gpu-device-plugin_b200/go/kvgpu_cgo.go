@@ -421,3 +421,81 @@ func revalidateBatchGPU(devs []string, want []string) (first int, err error) {
 	}
 	return -1, nil
 }
+
+// pluginDelta is what one rediscovery asks of the plugin servers (createDevicePlugins :131-137, :158-165).
+type pluginDelta struct {
+	Start, Stop, Resend []string // deviceMap keys ("%04x"); vGPU keys are returned by type id below
+	StartVgpu, StopVgpu, ResendVgpu []uint16
+}
+
+// rescanGPU: runtime rediscovery (SOURCE ONLY, unverified like the rest of this file).  The caller builds
+// snapshots in NUMERIC mode (addr = packed BDF, mdev uuid bytes, numeric groups and device ids, Walk order) and a
+// raw type dictionary that only grows at its end; the GPU diffs them against the previous rescan
+// (kvg_rescan_pci / kvg_rescan_mdev) and the key deltas become plugin actions: an added key starts a plugin, a
+// removed key stops it, a changed key re-sends its ListAndWatch list.  Changed iommuMap / gpuVgpuMap keys need no
+// plugin action: returnIommuMap / returnGpuVgpuMap read the rebuilt maps.  A snapshot that cannot be numeric
+// (interned names) must not come here: restart the plugins instead.  firstScan reports a missing baseline.
+func rescanGPU(pci []C.kvg_pci_rec, mdev []C.kvg_mdev_rec, dictOff []uint32, dictBytes []byte) (d pluginDelta, firstScan bool, err error) {
+	kvgMu.Lock()
+	defer kvgMu.Unlock()
+	if err := kvgEnsure(); err != nil {
+		return d, false, err
+	}
+	var pr *C.kvg_pci_rescan
+	var pp *C.kvg_pci_rec
+	if len(pci) > 0 {
+		pp = &pci[0]
+	}
+	if rc := C.kvg_rescan_pci(kvgCtx, pp, C.size_t(len(pci)), &pr); rc != C.KVG_OK {
+		return d, false, fmt.Errorf("kvg_rescan_pci: %s", C.GoString(C.kvg_last_error(kvgCtx)))
+	}
+	defer C.kvg_result_free(unsafe.Pointer(pr))
+	keys := func(k C.kvg_key_delta) (a, r, c []uint32) {
+		a = append(a, unsafe.Slice((*uint32)(unsafe.Pointer(k.added)), int(k.n_added))...)
+		r = append(r, unsafe.Slice((*uint32)(unsafe.Pointer(k.removed)), int(k.n_removed))...)
+		c = append(c, unsafe.Slice((*uint32)(unsafe.Pointer(k.changed)), int(k.n_changed))...)
+		return
+	}
+	a, r, c := keys(pr.dev)
+	hex := func(v []uint32) (out []string) {
+		for _, k := range v {
+			out = append(out, fmt.Sprintf("%04x", k))
+		}
+		return
+	}
+	d.Start, d.Stop, d.Resend = hex(a), hex(r), hex(c)
+	// the dictionary is copied into C memory: no Go pointer to Go memory crosses the call (cgo rule)
+	nt := len(dictOff) - 1
+	if nt < 0 {
+		nt = 0
+	}
+	cOff := (*C.uint32_t)(C.malloc(C.size_t(4 * (nt + 1))))
+	defer C.free(unsafe.Pointer(cOff))
+	cBytes := (*C.uint8_t)(C.malloc(C.size_t(len(dictBytes) + 1)))
+	defer C.free(unsafe.Pointer(cBytes))
+	offs := unsafe.Slice((*uint32)(unsafe.Pointer(cOff)), nt+1)
+	offs[0] = 0
+	copy(offs, dictOff)
+	copy(unsafe.Slice((*byte)(unsafe.Pointer(cBytes)), len(dictBytes)+1), dictBytes)
+	types := C.kvg_type_dict{n_types: C.uint32_t(nt), off: cOff, bytes: cBytes}
+	var mr *C.kvg_mdev_rescan
+	var mp *C.kvg_mdev_rec
+	if len(mdev) > 0 {
+		mp = &mdev[0]
+	}
+	if rc := C.kvg_rescan_mdev(kvgCtx, mp, C.size_t(len(mdev)), &types, &mr); rc != C.KVG_OK {
+		return d, false, fmt.Errorf("kvg_rescan_mdev: %s", C.GoString(C.kvg_last_error(kvgCtx)))
+	}
+	defer C.kvg_result_free(unsafe.Pointer(mr))
+	a, r, c = keys(mr._type)
+	for _, v := range a {
+		d.StartVgpu = append(d.StartVgpu, uint16(v))
+	}
+	for _, v := range r {
+		d.StopVgpu = append(d.StopVgpu, uint16(v))
+	}
+	for _, v := range c {
+		d.ResendVgpu = append(d.ResendVgpu, uint16(v))
+	}
+	return d, pr.had_baseline == 0 || mr.had_baseline == 0, nil
+}

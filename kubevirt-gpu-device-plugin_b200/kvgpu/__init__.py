@@ -5,8 +5,9 @@ package is the host-side mirror of the reference's plugin interface for that pat
 """
 from ._lib import (KVG_NO_NAME, MDEV_REC, MDEV_SURV, PCI_REC, PCI_SURV, KvgError, declared_symbols,
                    load)
-from .context import Context, HealthDelta, MdevResult, MdevShardResult, PciResult, PciShardResult
-from .plugin import (DiscoveryScan, Maps, MdevSnapshot, NvidiaGpuDevice, PciSnapshot, PluginSpec,
+from .context import (Context, HealthDelta, KeyDelta, MdevRescan, MdevResult, MdevShardResult, PciRescan, PciResult,
+                      PciShardResult)
+from .plugin import (DiscoveryScan, Maps, MdevSnapshot, NvidiaGpuDevice, PciSnapshot, PluginEvent, PluginSpec,
                      ReferencePanic, canonical_dump, format_bdf, format_uuid,
                      mdev_maps_from_result, parse_bdf, pci_maps_from_result, plugin_specs_from_maps,
                      snapshot_mdev_tree,

@@ -5,6 +5,8 @@ DevicePlugin server per device id / vGPU type, registered with the kubelet.
   python -m kvgpu --once --dump            scan, print the canonical dump, exit (no servers)
   python -m kvgpu --once --plugins         scan, print what each plugin would advertise (JSON)
   python -m kvgpu                          scan, serve, watch the device nodes, run until SIGTERM
+  python -m kvgpu --rediscover-period 5    the same, and rescan every 5 s: plugins start, stop and update
+                                           as devices and vGPUs appear, disappear or change
 
 There is no CPU fallback: without a usable CUDA device the scan fails and the process exits non-zero
 (the reference would log the failed walk and start no plugin)."""
@@ -26,6 +28,8 @@ def main(argv=None) -> int:
     ap.add_argument("--once", action="store_true", help="scan and print, do not serve")
     ap.add_argument("--dump", action="store_true", help="print the canonical dump of the five maps")
     ap.add_argument("--plugins", action="store_true", help="print the plugin specs as JSON")
+    ap.add_argument("--rediscover-period", type=float, default=0.0, metavar="SECONDS",
+                    help="rescan the trees this often and start / stop / update plugins (0: scan once)")
     args = ap.parse_args(argv)
 
     from . import DiscoveryScan, KvgError, canonical_dump
@@ -35,8 +39,11 @@ def main(argv=None) -> int:
         print("kvgpu: cannot create the scan context (no CPU fallback): %s" % e, file=sys.stderr)
         return 2
     try:
-        ds.create_iommu_device_map()      # :91
-        ds.create_vgpu_id_map()           # :93
+        if args.rediscover_period > 0 and not args.once:
+            ds.rediscover()               # the first rescan: maps + the baseline later rescans are diffed against
+        else:
+            ds.create_iommu_device_map()  # :91
+            ds.create_vgpu_id_map()       # :93
         specs = ds.create_device_plugins()
         if args.dump:
             sys.stdout.write(canonical_dump(ds.maps).decode("latin-1"))
@@ -62,10 +69,21 @@ def main(argv=None) -> int:
                 watchers.append(w)
             except Exception as e:        # noqa: BLE001
                 print("kvgpu: error starting the %s device plugin: %s" % (p.device_name, e), file=sys.stderr)
+        feed = None
+        if args.rediscover_period > 0:
+            live = {(s.vgpu, s.key): p for s, p in zip(specs, plugins) if p in started}
+            feed = serve.RediscoveryFeed(ds, live, args.rediscover_period, revalidate=reval, socket_dir=sockdir,
+                                         base_path=args.base_path, root_path=args.root_path,
+                                         vgpu_base_path=args.vgpu_base_path)
+            feed.watchers = {k: w for k, w in zip(live, watchers)}
+            feed.start()
         stop = threading.Event()
         for sig in (signal.SIGTERM, signal.SIGINT):
             signal.signal(sig, lambda *_: stop.set())
         stop.wait()                        # <-stop (:166)
+        if feed is not None:
+            feed.stop()                    # stops every watcher the feed holds
+            started, watchers = list(feed.plugins.values()), []
         for w in watchers:
             w.stop()
         for p in started:

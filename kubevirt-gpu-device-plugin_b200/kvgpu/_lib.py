@@ -98,6 +98,25 @@ class HealthDeltaC(C.Structure):
                 ("changed", C.c_void_p)]
 
 
+class KeyDeltaC(C.Structure):
+    _fields_ = [("n_added", C.c_uint32), ("added", C.c_void_p), ("n_removed", C.c_uint32),
+                ("removed", C.c_void_p), ("n_changed", C.c_uint32), ("changed", C.c_void_p)]
+
+
+class PciRescanC(C.Structure):
+    _fields_ = [("scan", PciResultC), ("had_baseline", C.c_uint32),
+                ("n_added", C.c_uint64), ("added", C.c_void_p), ("n_removed", C.c_uint64),
+                ("removed", C.c_void_p), ("n_moved", C.c_uint64), ("moved", C.c_void_p),
+                ("dev", KeyDeltaC), ("grp", KeyDeltaC)]
+
+
+class MdevRescanC(C.Structure):
+    _fields_ = [("scan", MdevResultC), ("had_baseline", C.c_uint32),
+                ("n_added", C.c_uint64), ("added", C.c_void_p), ("n_removed", C.c_uint64),
+                ("removed", C.c_void_p), ("n_moved", C.c_uint64), ("moved", C.c_void_p),
+                ("type", KeyDeltaC), ("parent", KeyDeltaC)]
+
+
 def declared_symbols() -> list[str]:
     """Every function name include/kvgpu.h declares (used by the export test)."""
     src = open(HEADER_PATH).read()
@@ -135,6 +154,9 @@ def load() -> C.CDLL:
         "kvg_scan_mdev": (C.c_int, [vp, vp, sz, P(TypeDict), P(P(MdevResultC))]),
         "kvg_health_rescan": (C.c_int, [vp, vp, sz, P(P(HealthDeltaC))]),
         "kvg_health_reset": (C.c_int, [vp]),
+        "kvg_rescan_pci": (C.c_int, [vp, vp, sz, P(P(PciRescanC))]),
+        "kvg_rescan_mdev": (C.c_int, [vp, vp, sz, P(TypeDict), P(P(MdevRescanC))]),
+        "kvg_rescan_reset": (C.c_int, [vp]),
         "kvg_text_pad": (sz, [sz]),
         "kvg_dev_pciids_parse": (C.c_int, [vp, vp, sz, sz, u32]),
         "kvg_dev_scan_pci": (C.c_int, [vp, vp, sz]),

@@ -71,6 +71,42 @@ class HealthDelta:
     changed: np.ndarray         # (index << 1) | now_alive
 
 
+@dataclass
+class KeyDelta:
+    """Key changes of one group-by map between two rescans (include/kvgpu.h kvg_key_delta); ascending."""
+    added: np.ndarray           # u32 keys absent before, present now
+    removed: np.ndarray         # u32 keys present before, absent now
+    changed: np.ndarray         # u32 keys present in both whose member list differs
+
+
+@dataclass
+class PciRescan:
+    """kvg_rescan_pci: the full scan plus its diff against the previous rescan."""
+    scan: PciResult
+    had_baseline: bool
+    added: np.ndarray           # indices into scan.survivors
+    removed: np.ndarray         # PCI_SURV, previous survivors
+    moved: np.ndarray           # indices into scan.survivors
+    dev: KeyDelta               # deviceMap
+    grp: KeyDelta               # iommuMap
+
+
+@dataclass
+class MdevRescan:
+    scan: MdevResult
+    had_baseline: bool
+    added: np.ndarray
+    removed: np.ndarray         # MDEV_SURV
+    moved: np.ndarray
+    type: KeyDelta              # vGpuMap (canonical type ids)
+    parent: KeyDelta            # gpuVgpuMap (parent handles)
+
+
+def _key_delta(k) -> KeyDelta:
+    return KeyDelta(L._arr(k.added, k.n_added, np.uint32), L._arr(k.removed, k.n_removed, np.uint32),
+                    L._arr(k.changed, k.n_changed, np.uint32))
+
+
 class _LockedLib:
     """A kvg_ctx is single-threaded (include/kvgpu.h).  gRPC handler threads, the health feed and the
     Allocate re-validation all share one Context (kvgpu/serve.py), so every C call on it is serialised."""
@@ -164,7 +200,7 @@ class Context:
                         [x.value for x in v]))
 
     # -- scans ------------------------------------------------------------------------------
-    def _take_pci(self, res) -> PciResult:
+    def _take_pci(self, res, free: bool = True) -> PciResult:
         r = res.contents
         S, KD, G = int(r.n_survivors), int(r.n_dev_keys), int(r.n_groups)
         dev_off = L._arr(r.dev_off, KD + 1, np.uint32)
@@ -181,7 +217,8 @@ class Context:
             grp_off=grp_off,
             grp_perm=L._arr(r.grp_perm, int(grp_off[-1]), np.uint32),
             name_pool=C.string_at(r.name_pool, r.name_pool_len) if r.name_pool_len else b"")
-        self._lib.kvg_result_free(res)
+        if free:
+            self._lib.kvg_result_free(res)
         return out
 
     def scan_pci(self, recs: np.ndarray) -> PciResult:
@@ -201,7 +238,7 @@ class Context:
                         blob.ctypes.data_as(C.POINTER(C.c_uint8)))
         return td, (off, blob)
 
-    def _take_mdev(self, res) -> MdevResult:
+    def _take_mdev(self, res, free: bool = True) -> MdevResult:
         r = res.contents
         S, KT, P, nt = int(r.n_survivors), int(r.n_type_keys), int(r.n_parents), int(r.n_types)
         loff = L._arr(r.label_off, nt + 1, np.uint32)
@@ -220,7 +257,8 @@ class Context:
             par_keys=L._arr(r.par_keys, P, np.uint32),
             par_off=L._arr(r.par_off, P + 1, np.uint32),
             par_perm=L._arr(r.par_perm, S, np.uint32))
-        self._lib.kvg_result_free(res)
+        if free:
+            self._lib.kvg_result_free(res)
         return out
 
     def scan_mdev(self, recs: np.ndarray, raw_types: list) -> MdevResult:
@@ -245,6 +283,35 @@ class Context:
 
     def health_reset(self):
         self._ck(self._lib.kvg_health_reset(self._h))
+
+    def rescan_pci(self, recs: np.ndarray) -> PciRescan:
+        """A full scan of `recs` (numeric mode, Walk order) diffed against the previous rescan."""
+        recs = np.ascontiguousarray(recs, dtype=L.PCI_REC)
+        res = C.POINTER(L.PciRescanC)()
+        self._ck(self._lib.kvg_rescan_pci(self._h, recs.ctypes.data, len(recs), C.byref(res)))
+        r = res.contents
+        out = PciRescan(self._take_pci(C.pointer(r.scan), free=False), bool(r.had_baseline),
+                        L._arr(r.added, r.n_added, np.uint32), L._arr(r.removed, r.n_removed, L.PCI_SURV),
+                        L._arr(r.moved, r.n_moved, np.uint32), _key_delta(r.dev), _key_delta(r.grp))
+        self._lib.kvg_result_free(res)
+        return out
+
+    def rescan_mdev(self, recs: np.ndarray, raw_types: list) -> MdevRescan:
+        """The same for mdevs; `raw_types` must extend the previous rescan's dictionary (append only)."""
+        recs = np.ascontiguousarray(recs, dtype=L.MDEV_REC)
+        td, keep = self._type_dict(raw_types)
+        res = C.POINTER(L.MdevRescanC)()
+        self._ck(self._lib.kvg_rescan_mdev(self._h, recs.ctypes.data, len(recs), C.byref(td), C.byref(res)))
+        del keep
+        r = res.contents
+        out = MdevRescan(self._take_mdev(C.pointer(r.scan), free=False), bool(r.had_baseline),
+                         L._arr(r.added, r.n_added, np.uint32), L._arr(r.removed, r.n_removed, L.MDEV_SURV),
+                         L._arr(r.moved, r.n_moved, np.uint32), _key_delta(r.type), _key_delta(r.parent))
+        self._lib.kvg_result_free(res)
+        return out
+
+    def rescan_reset(self):
+        self._ck(self._lib.kvg_rescan_reset(self._h))
 
     # -- device-resident entry points (raw device pointers, e.g. torch tensor.data_ptr()) ----
     def text_pad(self, n: int) -> int:

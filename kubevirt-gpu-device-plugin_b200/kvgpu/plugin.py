@@ -9,6 +9,8 @@ filter / join / bucketing run in libkvgpu.so on the GPU:
     DiscoveryScan.create_iommu_device_map    createIommuDeviceMap  (:187-247)
     DiscoveryScan.create_vgpu_id_map         createVgpuIDMap       (:255-291)
     DiscoveryScan.get_device_name            getDeviceName         (:371-422)
+    DiscoveryScan.rediscover                 a fresh snapshot diffed against the previous one on the GPU
+                                             (Context.rescan_pci / rescan_mdev) -> plugin start / stop / update
     DiscoveryScan.create_device_plugins      the payload half of createDevicePlugins (:99-157):
                                              per key the pluginapi.Device list, resource name,
                                              socket path and env key the Go servers would use
@@ -20,6 +22,7 @@ libkvgpu.so and a CUDA device DiscoveryScan cannot be constructed.
 from __future__ import annotations
 
 import os
+import threading
 from dataclasses import dataclass, field
 
 import numpy as np
@@ -338,6 +341,23 @@ class Maps:
     vGpuMap: dict = field(default_factory=dict)        # :65
     gpuVgpuMap: dict = field(default_factory=dict)     # :68
     deviceNames: dict = field(default_factory=dict)    # key -> getDeviceName(key) ("" = miss)
+    # held while the maps are swapped for a rediscovered set and while Allocate reads them
+    lock: threading.Lock = field(default_factory=threading.Lock, compare=False, repr=False)
+
+    def __getstate__(self):  # the maps travel between processes (sharded scans); the lock stays behind
+        state = dict(self.__dict__)
+        del state["lock"]
+        return state
+
+    def __setstate__(self, state):
+        self.__dict__.update(state)
+        self.lock = threading.Lock()
+
+    def swap(self, other: "Maps"):
+        """Take over `other`'s maps in one step with respect to readers holding `lock`."""
+        with self.lock:
+            self.iommuMap, self.deviceMap, self.bdfToIommuMap = other.iommuMap, other.deviceMap, other.bdfToIommuMap
+            self.vGpuMap, self.gpuVgpuMap, self.deviceNames = other.vGpuMap, other.gpuVgpuMap, other.deviceNames
 
 
 def pci_maps_from_result(res: PciResult, snap: PciSnapshot | None = None, maps: Maps | None = None,
@@ -436,6 +456,17 @@ class PluginSpec:
     vgpu: bool = False
 
 
+@dataclass
+class PluginEvent:
+    """What a rediscovery asks of the plugin servers: "start" a plugin for a new deviceMap / vGpuMap key,
+    "stop" the plugin of a removed key, "update" the device list of a changed key, or "replace_all" (stop
+    every plugin, start one per key of the new maps: what a restart of the plugin does)."""
+    kind: str
+    key: str | None = None
+    vgpu: bool = False
+    spec: PluginSpec | None = None
+
+
 class DiscoveryScan:
     """InitiateDevicePlugin's scan half (device_plugin.go:89-96) on the GPU."""
 
@@ -445,6 +476,8 @@ class DiscoveryScan:
         self.ctx = Context(device)
         self.maps = Maps()
         self._loaded_path = None
+        # rediscover(): the raw mdev type dictionary only ever grows, so canonical type ids stay stable
+        self._raw_types, self._type_index = [], {}
 
     def close(self):
         self.ctx.close()
@@ -452,6 +485,7 @@ class DiscoveryScan:
     def _ensure_table(self):
         if self._loaded_path == self.pciIdsFilePath:
             return
+        # (kvg_pciids_load drops the rescan baselines: the next rediscover() starts from "everything added")
         data = _read_file(self.pciIdsFilePath)
         # unreadable file -> getDeviceName returns "" for every key (:373-377): an empty table
         self.ctx.pciids_load(data if data is not None else b"")
@@ -478,6 +512,49 @@ class DiscoveryScan:
 
     def create_device_plugins(self) -> list:
         return plugin_specs_from_maps(self.maps)
+
+    def rediscover(self) -> list:
+        """Snapshot both trees again and bring self.maps up to date (in place, one swap).  Returns the
+        PluginEvents that take the plugin servers from the previous maps to the new ones.  Snapshots in
+        numeric mode go through the GPU diff; a snapshot in index mode has no stable identities and
+        yields [PluginEvent("replace_all")]."""
+        self._ensure_table()
+        psnap = snapshot_pci_tree(self.basePath)
+        msnap = snapshot_mdev_tree(self.vGpuBasePath, self.basePath)
+        remap = []
+        for raw in msnap.raw_types:
+            if raw not in self._type_index:
+                self._type_index[raw] = len(self._raw_types)
+                self._raw_types.append(raw)
+            remap.append(self._type_index[raw])
+        remap = np.array(remap, dtype=np.uint16)
+        recs = msnap.recs.copy()
+        if len(remap):
+            ok = (recs["flags"] & L.MF_TYPE_ERR) == 0
+            recs["type_idx"][ok] = remap[recs["type_idx"][ok]]
+        numeric = (psnap.packed_addr and psnap.group_names is None and psnap.device_names is None
+                   and msnap.uuid_ok and msnap.parent_names is None)
+        fresh = Maps()
+        if not numeric:
+            self.ctx.rescan_reset()
+            pci_maps_from_result(self.ctx.scan_pci(psnap.recs), psnap, fresh, name_of=self.ctx.name_lookup)
+            mdev_maps_from_result(self.ctx.scan_mdev(recs, self._raw_types), msnap, fresh)
+            self.maps.swap(fresh)
+            return [PluginEvent("replace_all")]
+        pr = self.ctx.rescan_pci(psnap.recs)
+        mr = self.ctx.rescan_mdev(recs, self._raw_types)
+        pci_maps_from_result(pr.scan, psnap, fresh, name_of=self.ctx.name_lookup)
+        mdev_maps_from_result(mr.scan, msnap, fresh)
+        self.maps.swap(fresh)
+        specs = {(s.vgpu, s.key): s for s in plugin_specs_from_maps(fresh)}
+        events = []
+        for vgpu, delta, key_of in ((False, pr.dev, lambda k: "%04x" % k),
+                                    (True, mr.type, lambda k: mr.scan.labels[k].decode("latin-1"))):
+            events += [PluginEvent("stop", key_of(int(k)), vgpu) for k in delta.removed]
+            events += [PluginEvent("start", key_of(int(k)), vgpu, specs[(vgpu, key_of(int(k)))]) for k in delta.added]
+            events += [PluginEvent("update", key_of(int(k)), vgpu, specs[(vgpu, key_of(int(k)))])
+                       for k in delta.changed]
+        return events
 
 
 def plugin_specs_from_maps(maps: Maps) -> list:

@@ -21,6 +21,7 @@ from __future__ import annotations
 
 import os
 import queue
+import sys
 import threading
 import time
 from concurrent import futures
@@ -31,7 +32,7 @@ import numpy as np
 from . import _lib as L
 from . import dpapi
 from .plugin import (DEVICE_NAMESPACE, GPU_PREFIX, VGPU_PREFIX, Maps, PluginSpec, ReferencePanic, _read_id,
-                     _read_link, _read_vgpu_raw)
+                     _read_link, _read_vgpu_raw, plugin_specs_from_maps)
 
 VFIO_DEVICE_PATH = "/dev/vfio"      # generic_device_plugin.go:54
 IOMMU_DEVICE_PATH = "/dev/iommu"    # :55
@@ -263,6 +264,12 @@ class _PluginBase:
     def unhealthy(self, dev_id: str):
         self._events.put(("unhealthy", dev_id))
 
+    def set_devices(self, devs: list):
+        """A rediscovery changed what this plugin advertises: ListAndWatch re-sends the whole new list."""
+        with self._lock:
+            self.devs = list(devs)
+        self._events.put(("devices", None))
+
     def resource_name(self) -> str:
         return "%s/%s" % (DEVICE_NAMESPACE, self.device_name)
 
@@ -286,10 +293,12 @@ class _PluginBase:
             except queue.Empty:
                 continue
             with self._lock:
-                for dev in self.devs:
-                    if dev.ID == dev_id:
-                        dev.health = dpapi.HEALTHY if kind == "healthy" else dpapi.UNHEALTHY
-            yield dpapi.ListAndWatchResponse(devices=self.devs)
+                if kind != "devices":        # "devices": set_devices replaced the whole list
+                    for dev in self.devs:
+                        if dev.ID == dev_id:
+                            dev.health = dpapi.HEALTHY if kind == "healthy" else dpapi.UNHEALTHY
+                devs = self.devs
+            yield dpapi.ListAndWatchResponse(devices=devs)
 
     # -- lifecycle
     def _handlers(self):
@@ -406,7 +415,8 @@ class GenericDevicePlugin(_PluginBase):
                     seen.add(host_path)
                     specs.append(dpapi.DeviceSpec(host_path=host_path, container_path=host_path, permissions="mrw"))
 
-            iommu_map, bdf_to_iommu = self.maps.iommuMap, self.maps.bdfToIommuMap
+            with self.maps.lock:           # a rediscovery swaps both maps together (Maps.swap)
+                iommu_map, bdf_to_iommu = self.maps.iommuMap, self.maps.bdfToIommuMap
             # plan: which devices would be visited, in order, and where a lookup error would stop
             plan, lookup_error_at = [], None
             for k, bdf in enumerate(req.devices_ids):
@@ -547,6 +557,85 @@ class HealthRescanFeed:
         self._stop.set()
         if self._thread:
             self._thread.join(2.0)
+
+
+# ------------------------------------------------------------------------------------------------
+# runtime rediscovery: GPU-diffed rescans start, stop and update plugins
+# ------------------------------------------------------------------------------------------------
+class RediscoveryFeed:
+    """Every `period_s`: ds.rediscover() (DiscoveryScan) and apply its PluginEvents to `plugins`, a dict
+    (vgpu, key) -> plugin shared with the caller.  start: build, start (register with the kubelet) and watch
+    a plugin; stop: stop it; update: replace its device list, which ListAndWatch re-sends whole;
+    replace_all: stop everything and start one plugin per key of the new maps.  `plugin_kw` are the
+    keyword arguments of plugins_from_specs (socket_dir, base_path, ...); `revalidate` goes to passthrough
+    plugins."""
+
+    def __init__(self, ds, plugins: dict, period_s: float, revalidate=None, watch: bool = True, **plugin_kw):
+        self.ds, self.plugins, self.period_s = ds, plugins, period_s
+        self.revalidate, self.watch, self.plugin_kw = revalidate, watch, plugin_kw
+        self.watchers = {}
+        self._stop = threading.Event()
+        self._thread = None
+
+    def _start(self, spec):
+        plugin = plugins_from_specs([spec], self.ds.maps, self.revalidate, **self.plugin_kw)[0]
+        plugin.start()
+        self.plugins[(spec.vgpu, spec.key)] = plugin
+        if self.watch:
+            w = DeviceNodeWatcher(plugin)
+            w.start()
+            self.watchers[(spec.vgpu, spec.key)] = w
+
+    def _stop_one(self, k):
+        w = self.watchers.pop(k, None)
+        if w is not None:
+            w.stop()
+        p = self.plugins.pop(k, None)
+        if p is not None:
+            p.stop()
+
+    def tick(self) -> list:
+        events = self.ds.rediscover()
+        for ev in events:
+            k = (ev.vgpu, ev.key)
+            try:
+                if ev.kind == "replace_all":
+                    for old in list(self.plugins):
+                        self._stop_one(old)
+                    for spec in plugin_specs_from_maps(self.ds.maps):
+                        self._start(spec)
+                elif ev.kind == "stop":
+                    self._stop_one(k)
+                elif ev.kind == "update" or (ev.kind == "start" and k in self.plugins):
+                    self.plugins[k].set_devices(devices_from_spec(ev.spec))
+                    if k in self.watchers:   # the watcher maps device nodes through the previous bdfToIommuMap
+                        self.watchers.pop(k).stop()
+                        w = DeviceNodeWatcher(self.plugins[k])
+                        w.start()
+                        self.watchers[k] = w
+                else:
+                    self._start(ev.spec)
+            except Exception as e:        # noqa: BLE001  a failed start is logged, the rest go on (:131-137)
+                print("kvgpu: rediscovery: %s %s: %s" % (ev.kind, ev.key, e), file=sys.stderr)
+        return events
+
+    def start(self):
+        def loop():
+            while not self._stop.wait(self.period_s):
+                try:
+                    self.tick()
+                except Exception as e:    # noqa: BLE001  a failed tick keeps the current plugins
+                    print("kvgpu: rediscovery failed: %s" % e, file=sys.stderr)
+        self._thread = threading.Thread(target=loop, daemon=True)
+        self._thread.start()
+
+    def stop(self):
+        self._stop.set()
+        if self._thread:
+            self._thread.join(5.0)
+        for w in self.watchers.values():
+            w.stop()
+        self.watchers.clear()
 
 
 # ------------------------------------------------------------------------------------------------
